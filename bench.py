@@ -11,7 +11,8 @@ per GPU (default 32 = BASELINE.json configs[1]).  metric = points/sec = GPUs * B
 One JSON line on stdout (rank 0).  `value`: inputs resident in HBM.  `e2e`: the step's depth maps
 and `choose` indices come from pinned host memory (H2D inside the timed region), are back-projected
 on the device, and a result digest is read back (D2H inside).  Other flags: --batch, --n-points, --k
-(stress sweep), --layout, --streams / --gather-streams (graph branches), --no-graph, --per-op.  `roofline`: the dominant kernel, per-op CUDA events on the launching stream
+(stress sweep), --layout, --streams / --gather-streams (graph branches), --no-graph, --per-op, --dump-outputs DIR
+(what the last timed step returned, as .npy files, to compare two builds output for output).  `roofline`: the dominant kernel, per-op CUDA events on the launching stream
 inside the timed region, against MEASURED_PEAKS.json.  `cpu_baseline`: the reference's compiled
 KNN (oracle/_ref, nanoflann, OpenMP over the batch) + its torch gather expression on the host
 cores, bounded sample.
@@ -281,6 +282,31 @@ def kernel_family(op_name):
     return SELF_FAMILY if key.startswith("cld_nei") else NONSELF_FAMILY
 
 
+DUMP_BYTES = 60 << 20      # all dumped arrays together, .npy headers aside: under 64 MB
+
+
+def sample_outputs(inputs, outs, gathers):
+    """{name: numpy array} of what one pass returns: every tensor of `inputs` (index tensors, point sets, choose)
+    and the gather outputs as ``gather_<index key>``.  Float tensors become float32, integer tensors float64
+    (exact).  An array larger than its share of DUMP_BYTES is replaced by its elements (in the logical shape's
+    flat order) at positions drawn without replacement by a generator seeded with 0: the same positions for the
+    same shape, so that two runs with the same arguments can be compared element for element."""
+    import numpy as np
+    import torch
+    arrays = dict(inputs)
+    arrays.update({"gather_%s" % g[1]: t for g, t in zip(gathers, outs)})
+    share = DUMP_BYTES // len(arrays)
+    res = {}
+    for name, t in sorted(arrays.items()):
+        dtype = np.dtype(np.float32 if t.is_floating_point() else np.float64)
+        cap = share // dtype.itemsize
+        if t.numel() > cap:
+            pos = np.sort(np.random.default_rng(0).choice(t.numel(), cap, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(pos).to(t.device)]
+        res[name] = t.cpu().numpy().astype(dtype)
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -299,7 +325,12 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="time eager launches instead of CUDA graph replays")
     ap.add_argument("--per-op", action="store_true", help="also print the per-op table to stderr")
     ap.add_argument("--l2-fetch", type=int, default=0, help="experiment: cudaLimitMaxL2FetchGranularity (32/64/128 bytes)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0) as DIR/<name>.npy, float32 or float64, "
+                         "under 64 MB in all: a larger array is a fixed seeded sample of its elements")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)
@@ -389,12 +420,16 @@ def main():
     torch.cuda.synchronize()
     e0.record()
     for _ in range(args.steps):
-        run_resident()
+        last = run_resident()
     e1.record()
     torch.cuda.synchronize()
     barrier()
     launches = launches_per_step * args.steps
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in sample_outputs(*last, p.gathers).items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     resident_res = run_resident()          # untimed: the results the end-to-end path must reproduce
     torch.cuda.synchronize()
 

@@ -5,10 +5,10 @@ function cites the reference lines it follows (relative to /root/reference/ffb6d
 KNN and grid subsampling call the C restatements in liboracle.so (knn_oracle.c,
 grid_oracle.c); the gather ops are closed-form numpy selections.
 
-Pinned against the reference itself: tests/test_oracle_vs_ref.py compares every
-function here with the reference's own code (oracle/_ref + AST-extracted torch
-functions) when /root/reference is present, and tests/golden/ holds the reference's
-outputs on seeded inputs for boxes where it is not.
+Pinned against the reference itself: tests/golden/ holds the outputs of the
+reference's own code (oracle/_ref + AST-extracted torch functions) on seeded
+inputs, and tests/test_oracle_golden.py / tests/test_oracle_vs_ref.py compare every
+function here with them.
 """
 import ctypes as C
 import os

@@ -426,6 +426,71 @@ def pose_cases():
     return out
 
 
+def wrap_padded_frame(n):
+    """A frame padded with repeated pixels (np.pad 'wrap', ycb_dataset.py:230): duplicated points, exact KNN ties."""
+    fr = make_frame(11, n_points=n)
+    rs = np.random.RandomState(5)
+    keep = fr["choose"][0][: n * 5 // 8]
+    choose = np.pad(keep, (0, n - len(keep)), "wrap")[rs.permutation(n)]
+    return dict(fr, cld=fr["dpt_xyz"].reshape(-1, 3)[choose])
+
+
+def oracle_ref_cases():
+    """The reference's results on the seeded inputs of tests/test_oracle_vs_ref.py (and of the wrap-padded frame
+    of tests/test_gpu_pass.py).  Results those tests compare exactly are stored as sha256 digests.  A KNN result
+    is stored as the rows where it differs from the oracle's result on the same inputs (tie order), plus the
+    sha256 of the whole int64 array: the test rebuilds the reference's array from the oracle's and checks it."""
+    from oracle import cpu_oracle as O
+    cases = {}
+
+    def knn(name, sup, qry, k, want):
+        want = want.astype(np.int64)
+        got = O.knn_batch(sup, qry, k).astype(np.int64)
+        rows = np.argwhere((got != want).any(axis=2)).astype(np.int32)
+        cases[name + "/rows"] = rows
+        cases[name + "/vals"] = want[rows[:, 0], rows[:, 1]].astype(np.int32)
+        cases[name + "/sha256"] = np.array(sha(want))
+
+    for seed, S, Q, K in ((0, 500, 300, 16), (1, 2000, 100, 1), (2, 64, 64, 32), (3, 5, 9, 8), (4, 3000, 700, 4)):
+        rs = np.random.RandomState(seed)
+        sup = rs.randn(2, S, 3).astype(np.float32)
+        qry = rs.randn(2, Q, 3).astype(np.float32)
+        knn("random%d" % seed, sup, qry, K, R.knn_batch(sup, qry, K, omp=True))
+    cld = make_frame(9, n_points=3072)["cld"][None]
+    knn("surface", cld, cld, 16, R.knn_batch(cld, cld, 16))
+    for n in (4096, 40960, 131072):
+        fr = make_frame(21, n_points=n)
+        lvl1 = fr["cld"][None, : n // 4]
+        lvl2 = fr["cld"][None, : n // 16]
+        img = np.ascontiguousarray(fr["dpt_xyz"][::4, ::4].reshape(1, -1, 3))
+        for j, (sup, qry, k) in enumerate(((lvl1, lvl1, 16), (lvl2, img, 1), (img, lvl2, 32))):
+            knn("stress%d_%d" % (n, j), sup, qry, k, R.knn_batch(sup, qry, k))
+    n = 3072
+    sets = point_sets(wrap_padded_frame(n), n)
+    for key, s, q, k in knn_schedule(n):
+        knn("wrap_" + key, sets[s][None], sets[q][None], k, R.knn_search(sets[s][None], sets[q][None], k))
+
+    f = R.torch_functions()
+    g = torch.Generator().manual_seed(7)
+    feat = torch.randn(3, 17, 211, 1, generator=g)
+    idx = torch.randint(0, 211, (3, 50, 16), generator=g)
+    cases["torch/random_sample"] = np.array(sha(f["random_sample"](feat, idx).numpy()))
+    idx1 = torch.randint(0, 211, (3, 400, 1), generator=g)
+    cases["torch/nearest_interpolation"] = np.array(sha(f["nearest_interpolation"](feat, idx1).numpy()))
+    pc = torch.randn(2, 90, 6, generator=g)
+    nidx = torch.randint(0, 90, (2, 90, 16), generator=g)
+    cases["torch/gather_neighbour"] = np.array(sha(f["gather_neighbour"](pc, nidx).numpy()))
+
+    rs = np.random.RandomState(5)
+    pts = (rs.randn(4000, 3) * 0.5).astype(np.float32)
+    feats = rs.rand(4000, 3).astype(np.float32)
+    rp, rf = R.grid_subsampling(pts, feats, None, 0.07)
+    o = np.lexsort((rp[:, 2], rp[:, 1], rp[:, 0]))
+    cases["grid/points"] = np.array(sha(rp[o]))
+    cases["grid/features"] = np.array(sha(rf[o]))
+    return cases
+
+
 def main():
     if not R.reference_sources_present():
         raise SystemExit("needs /root/reference")
@@ -433,7 +498,7 @@ def main():
     if len(sys.argv) > 2 and sys.argv[1] == "--only":      # regenerate one fixture file
         which = sys.argv[2]
         fn = {"lfa": lfa_cases, "knn": knn_cases, "gather": gather_cases, "grid": grid_cases, "train": train_cases,
-              "fusion": fusion_cases, "pose": pose_cases}[which]
+              "fusion": fusion_cases, "pose": pose_cases, "oracle_ref": oracle_ref_cases}[which]
         np.savez_compressed(os.path.join(OUT, which + "_cases.npz"), **fn())
         print("rewrote", which + "_cases.npz")
         return
@@ -444,6 +509,7 @@ def main():
     np.savez_compressed(os.path.join(OUT, "fusion_cases.npz"), **fusion_cases())
     np.savez_compressed(os.path.join(OUT, "train_cases.npz"), **train_cases())
     np.savez_compressed(os.path.join(OUT, "pose_cases.npz"), **pose_cases())
+    np.savez_compressed(os.path.join(OUT, "oracle_ref_cases.npz"), **oracle_ref_cases())
     dig = {"generator": "ffb6d_b200.synthetic.make_frame", "frames": {}}
     for seed, n in ((0, 12288), (1, 12288), (2, 3072)):
         dig["frames"]["seed%d_n%d" % (seed, n)] = {"seed": seed, "n_points": n,

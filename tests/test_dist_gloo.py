@@ -54,6 +54,12 @@ def test_reference_arm_prints_on_rank0_only():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_steps_must_be_positive():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                         capture_output=True, text=True, timeout=300)
+    assert out.returncode == 2 and "--steps" in out.stderr
+
+
 def test_reference_arm_line_shape():
     env = dict(os.environ, RANK="0", WORLD_SIZE="1")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",

@@ -105,6 +105,32 @@ def test_e2e_graph_from_depth_equals_resident(cuda, batch32):
             assert torch.equal(g, w)
 
 
+def test_bench_dump_outputs_are_the_timed_pass(cuda, tmp_path):
+    """bench.py --dump-outputs writes what its timed pass returns: the arrays of a pass over the same frames and
+    features run here, sampled the same way, under 64 MB in all."""
+    import subprocess
+    import sys
+    import bench
+    from conftest import ROOT
+    from ffb6d_b200.pipeline import FusionPass
+    from ffb6d_b200.synthetic import make_batch
+    B, n = 2, 3072
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--batch", str(B), "--n-points", str(n),
+                          "--steps", "2", "--warmup", "1", "--no-mlp", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=900)
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == 2
+    p = FusionPass(B, n_points=n, device=cuda, seed=0)
+    want = bench.sample_outputs(*p(*_device_inputs(make_batch(range(B), n_points=n), cuda)), p.gathers)
+    files = sorted(os.listdir(tmp_path))
+    assert files == sorted(name + ".npy" for name in want)
+    assert sum(os.path.getsize(tmp_path / f) for f in files) <= 64 * 10 ** 6
+    for name, w in want.items():
+        got = np.load(tmp_path / (name + ".npy"))
+        assert got.dtype in (np.float32, np.float64) and got.dtype == w.dtype, name
+        assert np.array_equal(got, w), name
+
+
 def test_two_devices_in_one_process():
     """Per-device caches (shared-memory opt-in, SM count): ops on cuda:1 after cuda:0 in the same process."""
     if torch.cuda.device_count() < 2:
@@ -140,7 +166,7 @@ def test_index_validation(cuda):
     assert torch.isfinite(feat.grad).all()
 
 
-def test_wrap_padded_frame_downstream_features_unchanged(cuda):
+def test_wrap_padded_frame_downstream_features_unchanged(cuda, oracle_ref_golden):
     """The datasets pad frames with fewer valid pixels than points by repeating pixels (np.pad 'wrap',
     ycb_dataset.py:230): the cloud then holds duplicated points and KNN has exact distance ties, where our neighbour
     order (ascending index) differs from the reference's (KD-tree traversal order).  Duplicated points carry identical
@@ -162,11 +188,10 @@ def test_wrap_padded_frame_downstream_features_unchanged(cuda):
     for sr, pts in image_pyramid_np(fr["dpt_xyz"]).items():
         sets[("img", sr)] = pts
     ours = F.build_ffb6d_indices(torch.from_numpy(cld)[None].cuda(), torch.from_numpy(fr["dpt_xyz"])[None].cuda())
-    # the reference's own compiled KNN (KD-tree traversal order under ties) where oracle/_ref travelled with the
-    # snapshot, else the restatement (same neighbour sets, our tie order)
-    from oracle import ref_loader as R
-    ref_knn = R.knn_search if R.knn_available() else O.knn_search
-    ref = {key: ref_knn(sets[s][None], sets[q][None], kk) for key, s, q, kk in knn_schedule(n)}
+    # the reference's own compiled KNN (KD-tree traversal order under ties), stored in tests/golden
+    from conftest import reference_knn
+    ref = {key: reference_knn(oracle_ref_golden, "wrap_" + key, O.knn_search(sets[s][None], sets[q][None], kk))
+           for key, s, q, kk in knn_schedule(n)}
     ref.update({"cld_sub_idx%d" % i: ref["cld_nei_idx%d" % i][:, : n // 4 ** (i + 1)] for i in range(4)})
     n_tied = 0
     for key, s, q, kk in knn_schedule(n):
@@ -174,8 +199,7 @@ def test_wrap_padded_frame_downstream_features_unchanged(cuda):
         ok, _, _, msg = O.knn_matches(sets[s][None], sets[q][None], got, ref[key])
         assert ok, (key, msg)
         n_tied += int((got != ref[key]).any(axis=2).sum())
-    if R.knn_available():
-        assert n_tied > 0                                                # the tie order really differs somewhere
+    assert n_tied > 0                                                    # the tie order really differs somewhere
     calls = {key: (s, q) for key, s, q, kk in knn_schedule(n)}
     for op, key, C, S, Q, K in gather_schedule(n):
         if op == "choose":

@@ -1,36 +1,34 @@
-"""CPU, only where /root/reference exists (this container): the oracle against the
-reference's own code executed live on fresh random inputs."""
+"""CPU: the oracle against the reference's own code on seeded random inputs.  The reference's results on these
+inputs are stored in tests/golden/oracle_ref_cases.npz (tests/golden/make_golden.py)."""
 import numpy as np
 import pytest
 
+from conftest import reference_knn, sha256_of
 from oracle import cpu_oracle as O
-from oracle import ref_loader as R
-
-pytestmark = pytest.mark.skipif(not (R.reference_sources_present() and R.knn_available()),
-                                reason="reference sources / oracle/_ref not present on this box")
 
 
 @pytest.mark.parametrize("seed,S,Q,K", [(0, 500, 300, 16), (1, 2000, 100, 1), (2, 64, 64, 32),
                                         (3, 5, 9, 8), (4, 3000, 700, 4)])
-def test_knn_random(seed, S, Q, K):
+def test_knn_random(oracle_ref_golden, seed, S, Q, K):
     rs = np.random.RandomState(seed)
     sup = rs.randn(2, S, 3).astype(np.float32)
     qry = rs.randn(2, Q, 3).astype(np.float32)
-    want = R.knn_batch(sup, qry, K, omp=True)
     got = O.knn_batch(sup, qry, K)
+    want = reference_knn(oracle_ref_golden, "random%d" % seed, got)
     ok, ndiff, _, msg = O.knn_matches(sup, qry, got, want)
     assert ok and ndiff == 0, msg
 
 
-def test_knn_surface_frame():
+def test_knn_surface_frame(oracle_ref_golden):
     from ffb6d_b200.synthetic import make_frame
     fr = make_frame(9, n_points=3072)
     cld = fr["cld"][None]
-    assert np.array_equal(O.knn_batch(cld, cld, 16), R.knn_batch(cld, cld, 16))
+    got = O.knn_batch(cld, cld, 16)
+    assert np.array_equal(got, reference_knn(oracle_ref_golden, "surface", got))
 
 
 @pytest.mark.parametrize("n_points", [4096, 40960, 131072])
-def test_knn_stress_sweep_sizes(n_points):
+def test_knn_stress_sweep_sizes(oracle_ref_golden, n_points):
     """BASELINE configs[4] sizes: the port still equals the reference's KD-tree on the big clouds
     (self search K = 16 on level 1, image -> cloud K = 1 and cloud -> image K = 32 on level 2)."""
     from ffb6d_b200.synthetic import make_frame
@@ -40,42 +38,42 @@ def test_knn_stress_sweep_sizes(n_points):
     img = np.ascontiguousarray(fr["dpt_xyz"][::4, ::4].reshape(1, -1, 3))
     # dense clouds do produce the odd exact fp32 distance tie (seen: one row of 10240 at N0 = 40960), and
     # the hole pixels of the image level are exact duplicates: rows may then differ in ORDER only
-    for sup, qry, k in ((lvl1, lvl1, 16), (lvl2, img, 1), (img, lvl2, 32)):
-        got, want = O.knn_batch(sup, qry, k), R.knn_batch(sup, qry, k)
+    for j, (sup, qry, k) in enumerate(((lvl1, lvl1, 16), (lvl2, img, 1), (img, lvl2, 32))):
+        got = O.knn_batch(sup, qry, k)
+        want = reference_knn(oracle_ref_golden, "stress%d_%d" % (n_points, j), got)
         ok, ndiff, nties, msg = O.knn_matches(sup, qry, got, want)
         assert ok and ndiff == nties, msg
         assert ndiff <= max(4, got.shape[1] // 1000) or sup is img, msg
 
 
-def test_torch_ops_random():
+def test_torch_ops_random(oracle_ref_golden):
     import torch
-    f = R.torch_functions()
+    want = oracle_ref_golden["torch"]
     g = torch.Generator().manual_seed(7)
     feat = torch.randn(3, 17, 211, 1, generator=g)
     idx = torch.randint(0, 211, (3, 50, 16), generator=g)
-    assert np.array_equal(f["random_sample"](feat, idx).numpy(), O.random_sample(feat.numpy(), idx.numpy()))
+    got = O.random_sample(feat.numpy(), idx.numpy())
+    assert got.shape == (3, 17, 50, 1) and sha256_of(got) == str(want["random_sample"])
     idx1 = torch.randint(0, 211, (3, 400, 1), generator=g)
-    assert np.array_equal(f["nearest_interpolation"](feat, idx1).numpy(),
-                          O.nearest_interpolation(feat.numpy(), idx1.numpy()))
+    got = O.nearest_interpolation(feat.numpy(), idx1.numpy())
+    assert got.shape == (3, 17, 400, 1) and sha256_of(got) == str(want["nearest_interpolation"])
     pc = torch.randn(2, 90, 6, generator=g)
     nidx = torch.randint(0, 90, (2, 90, 16), generator=g)
-    assert np.array_equal(f["gather_neighbour"](pc, nidx).numpy(),
-                          O.gather_neighbour(pc.numpy(), nidx.numpy()))
+    got = O.gather_neighbour(pc.numpy(), nidx.numpy())
+    assert got.shape == (2, 90, 16, 6) and sha256_of(got) == str(want["gather_neighbour"])
 
 
-@pytest.mark.skipif(not R.grid_available(), reason="oracle/_ref/libgrid_ref.so missing")
-def test_grid_random():
+def test_grid_random(oracle_ref_golden):
     rs = np.random.RandomState(5)
     pts = (rs.randn(4000, 3) * 0.5).astype(np.float32)
     feats = rs.rand(4000, 3).astype(np.float32)
-    rp, rf = R.grid_subsampling(pts, feats, None, 0.07)
     op, of, _ = O.grid_sub_sampling(pts, feats, None, 0.07)
-    o1 = np.lexsort((rp[:, 2], rp[:, 1], rp[:, 0]))
-    o2 = np.lexsort((op[:, 2], op[:, 1], op[:, 0]))
-    assert np.array_equal(rp[o1], op[o2]) and np.array_equal(rf[o1], of[o2])
+    o = np.lexsort((op[:, 2], op[:, 1], op[:, 0]))
+    assert sha256_of(op[o]) == str(oracle_ref_golden["grid"]["points"])
+    assert sha256_of(of[o]) == str(oracle_ref_golden["grid"]["features"])
 
 
-def test_wrap_padded_frame_tie_order_differs_but_gathers_agree():
+def test_wrap_padded_frame_tie_order_differs_but_gathers_agree(oracle_ref_golden):
     """A frame padded with repeated pixels (np.pad 'wrap', ycb_dataset.py:230): thousands of index rows differ
     between the reference's KD-tree order and the (distance, index) order -- within the tie contract -- yet every
     gather of the forward pass returns the same values, because tied points are duplicates with identical features."""
@@ -91,8 +89,8 @@ def test_wrap_padded_frame_tie_order_differs_but_gathers_agree():
     sets = frame_point_sets(fr, n)
     ref, ours, differing = {}, {}, 0
     for key, s, q, kk in knn_schedule(n):
-        ref[key] = R.knn_search(sets[s][None], sets[q][None], kk)
         ours[key] = O.knn_search(sets[s][None], sets[q][None], kk)
+        ref[key] = reference_knn(oracle_ref_golden, "wrap_" + key, ours[key])
         ok, _, _, msg = O.knn_matches(sets[s][None], sets[q][None], ours[key], ref[key])
         assert ok, (key, msg)
         differing += int((ref[key] != ours[key]).any(axis=2).sum())
