@@ -35,7 +35,7 @@ def _load():
             "%s not found: the CUDA library has not been built (run __graft_entry__.build() "
             "or `make -C ffb6d_b200/csrc`). There is no CPU fallback." % LIB_PATH)
     lib = C.CDLL(LIB_PATH)
-    vp, i64, sz, ci, fp = C.c_void_p, C.c_int64, C.c_size_t, C.c_int, C.c_float
+    vp, i64, sz, ci, fp, dp = C.c_void_p, C.c_int64, C.c_size_t, C.c_int, C.c_float, C.c_double
     sig = {
         "ffb6d_version": (ci, []),
         "ffb6d_last_error": (C.c_char_p, []),
@@ -71,6 +71,10 @@ def _load():
         "ffb6d_bn_workspace_bytes": (sz, [i64, i64]),
         "ffb6d_bn_train_fwd": (ci, [vp, i64, i64, i64, vp, vp, fp, fp, vp, vp, ci, fp, vp, vp, vp, sz, vp]),
         "ffb6d_bn_train_bwd": (ci, [vp, vp, vp, i64, i64, i64, ci, fp, vp, vp, vp, vp, sz, vp]),
+        "ffb6d_bn_train_stats": (ci, [vp, i64, i64, i64, vp, vp, sz, vp]),
+        "ffb6d_bn_train_apply": (ci, [vp, i64, i64, i64, vp, dp, vp, vp, fp, fp, vp, vp, ci, fp, vp, vp, vp]),
+        "ffb6d_bn_train_bwd_stats": (ci, [vp, vp, vp, i64, i64, i64, ci, fp, vp, vp, vp, vp, sz, vp]),
+        "ffb6d_bn_train_bwd_apply": (ci, [vp, vp, vp, vp, dp, i64, i64, i64, ci, fp, vp, vp]),
         "ffb6d_act_bwd": (ci, [vp, vp, i64, ci, fp, vp, vp]),
         "ffb6d_fusion_mlp_wgrad": (ci, [vp, vp, i64, vp, i64, i64, i64, i64, vp, vp]),
         "ffb6d_att_pool_bwd": (ci, [vp, i64, vp, i64, vp, vp, i64, i64, ci, vp, vp, vp, vp]),

@@ -195,6 +195,73 @@ bn_bwd_apply_kernel(const float *__restrict__ z, const float *__restrict__ g, co
     }
 }
 
+// ------------------------------------------------------------------ BatchNorm split at the reduction (SyncBatchNorm)
+// The entry points ffb6d_bn_train_{stats,apply,bwd_stats,bwd_apply} run the kernels above with the per-channel fp64
+// sums handed to the caller in between, so that they can be all-reduced across ranks.  Each kernel below repeats the
+// arithmetic of its single-GPU counterpart expression for expression: at one rank the split path is bit-identical.
+
+// sums[c] = (sum over s of partial[c][s]) in ascending s, as bn_finalize_kernel / bn_bwd_finalize_kernel add them;
+// with grad_beta / grad_gamma, also their float roundings (the local dbeta, dgamma)
+__global__ void __launch_bounds__(BN_THREADS)
+bn_partial_sums_kernel(const double *__restrict__ partial, int C, int nsplit, double *__restrict__ sums,
+                       float *__restrict__ grad_gamma, float *__restrict__ grad_beta)
+{
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= C) return;
+    double A = 0.0, Q = 0.0;
+    for (int s = 0; s < nsplit; ++s) {
+        A += partial[((size_t)c * nsplit + s) * 2];
+        Q += partial[((size_t)c * nsplit + s) * 2 + 1];
+    }
+    sums[2 * (size_t)c] = A;
+    sums[2 * (size_t)c + 1] = Q;
+    if (grad_beta) grad_beta[c] = (float)A;
+    if (grad_gamma) grad_gamma[c] = (float)Q;
+}
+
+// bn_finalize_kernel with the partials already added up (sums[c] = (sum z, sum z^2) over n elements of all ranks)
+__global__ void __launch_bounds__(BN_THREADS)
+bn_finalize_sums_kernel(const double *__restrict__ sums, int C, double n, float eps, float momentum,
+                        const float *__restrict__ gamma, const float *__restrict__ beta, float *__restrict__ running_mean,
+                        float *__restrict__ running_var, float4 *__restrict__ stats)
+{
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= C) return;
+    const double A = sums[2 * (size_t)c], Q = sums[2 * (size_t)c + 1];
+    const double mean = A / n;
+    double var = Q / n - mean * mean;
+    if (var < 0.0) var = 0.0;
+    const float invstd = (float)(1.0 / sqrt(var + (double)eps));
+    const float g = gamma ? gamma[c] : 1.f;
+    stats[c] = make_float4((float)mean, invstd, g * invstd, beta ? beta[c] : 0.f);
+    if (running_mean) running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * (float)mean;
+    if (running_var) {
+        const double unbiased = n > 1.0 ? var * n / (n - 1.0) : var;
+        running_var[c] = (1.f - momentum) * running_var[c] + momentum * (float)unbiased;
+    }
+}
+
+// bn_bwd_apply_kernel reading the fp64 sums (sum g', sum g' * xhat) of all ranks, rounded to float as
+// bn_bwd_finalize_kernel rounds them
+__global__ void __launch_bounds__(BN_THREADS)
+bn_bwd_apply_sums_kernel(const float *__restrict__ z, const float *__restrict__ g, const float4 *__restrict__ stats,
+                         const double *__restrict__ sums, int C, int P, float inv_n, int act, float slope,
+                         float *__restrict__ dz)
+{
+    const size_t row = blockIdx.x;
+    const int c = (int)(row % C);
+    const float4 st = stats[c];
+    const float2 sm = make_float2((float)sums[2 * (size_t)c], (float)sums[2 * (size_t)c + 1]);
+    const float mb = sm.x * inv_n, mg = sm.y * inv_n;
+    const float *zr = z + row * P, *gr = g + row * P;
+    float *dr = dz + row * P;
+    for (int p = blockIdx.y * BN_THREADS + threadIdx.x; p < P; p += BN_THREADS * gridDim.y) {
+        const float d = __ldg(zr + p) - st.x;
+        const float gp = act_grad(__ldg(gr + p), __fmaf_rn(d, st.z, st.w), act, slope);
+        dr[p] = st.z * (gp - mb - (d * st.y) * mg);
+    }
+}
+
 // activation backward alone (a layer without BatchNorm but with an activation): dz = g * act'(z)
 __global__ void __launch_bounds__(BN_THREADS)
 act_bwd_kernel(const float *__restrict__ z, const float *__restrict__ g, long long n, int act, float slope, float *__restrict__ dz)
@@ -428,6 +495,96 @@ int ffb6d_bn_train_bwd(const float *z, const float *grad_y, const float *stats, 
     FFB6D_LAUNCH_OK("bn_bwd_apply_kernel");
     return FFB6D_OK;
 }
+
+#define FFB6D_BN_SIZES_OK(who)                                                                                           \
+    FFB6D_CHECK_ARG(B >= 1 && C >= 1 && P >= 1 && B < 65536 && C <= 65535 && P < (1ll << 31) && B * C < (1ll << 31), \
+                    who ": bad size")
+#define FFB6D_BN_COUNT_OK(who)                                                                                   \
+    FFB6D_CHECK_ARG(count >= (double)B * (double)P && count < 9.007199254740992e15, who ": count %g outside [B*P = %lld, 2^53)", \
+                    count, (long long)(B * P))
+
+int ffb6d_bn_train_stats(const float *z, int64_t B, int64_t C, int64_t P, double *sums, void *workspace,
+                         size_t workspace_bytes, ffb6d_stream_t stream)
+{
+    FFB6D_BN_SIZES_OK("bn_train_stats");
+    FFB6D_CHECK_ARG(z && sums && workspace, "bn_train_stats: null pointer");
+    FFB6D_CHECK_ARG((reinterpret_cast<uintptr_t>(sums) & 7) == 0, "bn_train_stats: sums must be 8-byte aligned");
+    FFB6D_CHECK_ARG(workspace_bytes >= ffb6d_bn_workspace_bytes(C, P), "bn_train_stats: workspace too small");
+    cudaStream_t st = (cudaStream_t)stream;
+    int chunk, nsplit;
+    split_plan(C, P, chunk, nsplit);
+    double *partial = (double *)workspace;
+    bn_stats_kernel<<<dim3((unsigned)nsplit, (unsigned)C), BN_THREADS, 0, st>>>(z, (int)B, (int)C, (int)P, chunk, nsplit, partial);
+    FFB6D_LAUNCH_OK("bn_stats_kernel");
+    bn_partial_sums_kernel<<<(unsigned)ceil_div(C, BN_THREADS), BN_THREADS, 0, st>>>(partial, (int)C, nsplit, sums, nullptr,
+                                                                                    nullptr);
+    FFB6D_LAUNCH_OK("bn_partial_sums_kernel");
+    return FFB6D_OK;
+}
+
+int ffb6d_bn_train_apply(const float *z, int64_t B, int64_t C, int64_t P, const double *sums, double count,
+                         const float *gamma, const float *beta, float eps, float momentum, float *running_mean,
+                         float *running_var, int act, float negative_slope, float *stats, float *y, ffb6d_stream_t stream)
+{
+    FFB6D_BN_SIZES_OK("bn_train_apply");
+    FFB6D_CHECK_ARG(z && sums && stats && y, "bn_train_apply: null pointer");
+    FFB6D_CHECK_ARG(act >= 0 && act <= 2, "bn_train_apply: act=%d", act);
+    FFB6D_BN_COUNT_OK("bn_train_apply");
+    FFB6D_CHECK_ARG((reinterpret_cast<uintptr_t>(sums) & 7) == 0, "bn_train_apply: sums must be 8-byte aligned");
+    FFB6D_CHECK_ARG((reinterpret_cast<uintptr_t>(stats) & 15) == 0, "bn_train_apply: stats must be 16-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    bn_finalize_sums_kernel<<<(unsigned)ceil_div(C, BN_THREADS), BN_THREADS, 0, st>>>(
+        sums, (int)C, count, eps, momentum, gamma, beta, running_mean, running_var, (float4 *)stats);
+    FFB6D_LAUNCH_OK("bn_finalize_sums_kernel");
+    const unsigned gx = (unsigned)std::min<int64_t>(ceil_div(P, 4 * BN_THREADS), 64);
+    bn_apply_kernel<<<dim3((unsigned)(B * C), gx), BN_THREADS, 0, st>>>(z, (const float4 *)stats, (int)C, (int)P, act,
+                                                                        negative_slope, y);
+    FFB6D_LAUNCH_OK("bn_apply_kernel");
+    return FFB6D_OK;
+}
+
+int ffb6d_bn_train_bwd_stats(const float *z, const float *grad_y, const float *stats, int64_t B, int64_t C, int64_t P,
+                             int act, float negative_slope, double *sums, float *grad_gamma, float *grad_beta,
+                             void *workspace, size_t workspace_bytes, ffb6d_stream_t stream)
+{
+    FFB6D_BN_SIZES_OK("bn_train_bwd_stats");
+    FFB6D_CHECK_ARG(z && grad_y && stats && sums && workspace, "bn_train_bwd_stats: null pointer");
+    FFB6D_CHECK_ARG(act >= 0 && act <= 2, "bn_train_bwd_stats: act=%d", act);
+    FFB6D_CHECK_ARG((reinterpret_cast<uintptr_t>(sums) & 7) == 0, "bn_train_bwd_stats: sums must be 8-byte aligned");
+    FFB6D_CHECK_ARG((reinterpret_cast<uintptr_t>(stats) & 15) == 0, "bn_train_bwd_stats: stats must be 16-byte aligned");
+    FFB6D_CHECK_ARG(workspace_bytes >= ffb6d_bn_workspace_bytes(C, P), "bn_train_bwd_stats: workspace too small");
+    cudaStream_t st = (cudaStream_t)stream;
+    int chunk, nsplit;
+    split_plan(C, P, chunk, nsplit);
+    double *partial = (double *)workspace;
+    bn_bwd_reduce_kernel<<<dim3((unsigned)nsplit, (unsigned)C), BN_THREADS, 0, st>>>(
+        z, grad_y, (const float4 *)stats, (int)B, (int)C, (int)P, chunk, nsplit, act, negative_slope, partial);
+    FFB6D_LAUNCH_OK("bn_bwd_reduce_kernel");
+    bn_partial_sums_kernel<<<(unsigned)ceil_div(C, BN_THREADS), BN_THREADS, 0, st>>>(partial, (int)C, nsplit, sums, grad_gamma,
+                                                                                    grad_beta);
+    FFB6D_LAUNCH_OK("bn_partial_sums_kernel");
+    return FFB6D_OK;
+}
+
+int ffb6d_bn_train_bwd_apply(const float *z, const float *grad_y, const float *stats, const double *sums, double count,
+                             int64_t B, int64_t C, int64_t P, int act, float negative_slope, float *grad_z,
+                             ffb6d_stream_t stream)
+{
+    FFB6D_BN_SIZES_OK("bn_train_bwd_apply");
+    FFB6D_CHECK_ARG(z && grad_y && stats && sums && grad_z, "bn_train_bwd_apply: null pointer");
+    FFB6D_CHECK_ARG(act >= 0 && act <= 2, "bn_train_bwd_apply: act=%d", act);
+    FFB6D_BN_COUNT_OK("bn_train_bwd_apply");
+    FFB6D_CHECK_ARG((reinterpret_cast<uintptr_t>(sums) & 7) == 0, "bn_train_bwd_apply: sums must be 8-byte aligned");
+    FFB6D_CHECK_ARG((reinterpret_cast<uintptr_t>(stats) & 15) == 0, "bn_train_bwd_apply: stats must be 16-byte aligned");
+    const unsigned gx = (unsigned)std::min<int64_t>(ceil_div(P, BN_THREADS), 64);
+    bn_bwd_apply_sums_kernel<<<dim3((unsigned)(B * C), gx), BN_THREADS, 0, (cudaStream_t)stream>>>(
+        z, grad_y, (const float4 *)stats, sums, (int)C, (int)P, (float)(1.0 / count), act, negative_slope, grad_z);
+    FFB6D_LAUNCH_OK("bn_bwd_apply_sums_kernel");
+    return FFB6D_OK;
+}
+
+#undef FFB6D_BN_SIZES_OK
+#undef FFB6D_BN_COUNT_OK
 
 int ffb6d_act_bwd(const float *z, const float *grad_y, int64_t n, int act, float negative_slope, float *grad_z,
                   ffb6d_stream_t stream)

@@ -18,8 +18,19 @@ Both modes run on the CUDA library:
 
 A layer accepts its input as one tensor or as the two halves of a concat (``layer(x1, x2)`` ==
 ``layer(torch.cat((x1, x2), 1))`` without materialising the concat, models/ffb6d.py:251-262).
+
+Synchronised BatchNorm: the reference trains with every BatchNorm converted to SyncBN (train_ycb.py:568).
+``torch.nn.SyncBatchNorm.convert_sync_batchnorm(model)`` works on these modules and keeps the state-dict keys.
+A layer whose ``bn`` child is an ``nn.SyncBatchNorm`` then decides like torch does: in training mode, with
+``torch.distributed`` initialised and more than one rank in ``bn.process_group`` (default WORLD), it normalises
+with the statistics of the global batch -- one all-reduce of the fp64 per-channel sums and the local element
+count in the forward (``ffb6d_bn_train_stats`` / ``_apply``), one in the backward (``ffb6d_bn_train_bwd_stats`` /
+``_bwd_apply``); the global count is read back to the host, one synchronisation per layer.  Running statistics
+come out identical on every rank; gamma / beta gradients are the local sums, which DDP averages.  Every rank
+needs at least one frame.  Otherwise (eval mode, one rank, no process group) the layer runs exactly as unconverted.
 """
 import torch
+import torch.distributed as dist
 import torch.nn as nn
 import torch.nn.functional as F_
 
@@ -56,10 +67,12 @@ def _gemm(x1, x2, w2d):
 
 
 class _ConvBnActTrain(torch.autograd.Function):
-    """conv1x1(cat(x1, x2)) -> [BatchNorm with batch statistics] -> activation, with its backward."""
+    """conv1x1(cat(x1, x2)) -> [BatchNorm with batch statistics] -> activation, with its backward.
+    ``group``: a process group to take the BatchNorm statistics over (SyncBatchNorm), or None for this rank's."""
 
     @staticmethod
-    def forward(ctx, x1, x2, weight, bias, gamma, beta, running_mean, running_var, eps, momentum, act, slope, has_bn):
+    def forward(ctx, x1, x2, weight, bias, gamma, beta, running_mean, running_var, eps, momentum, act, slope, has_bn,
+                group=None):
         x1 = x1.contiguous()
         x2 = x2.contiguous() if x2 is not None else None
         B, C1 = x1.shape[0], x1.shape[1]
@@ -72,19 +85,31 @@ class _ConvBnActTrain(torch.autograd.Function):
         else:
             z = _gemm(x1, x2, w2d)
         P = z.numel() // (B * Co)
-        stats = None
+        stats = count = None
         if has_bn:
             stats = torch.empty((Co, 4), dtype=torch.float32, device=z.device)
             y = torch.empty_like(z)
             nbytes = int(lib.ffb6d_bn_workspace_bytes(Co, P))
             ws = torch.empty(nbytes, dtype=torch.uint8, device=z.device)
+            affine = (gamma.data_ptr() if gamma is not None else None, beta.data_ptr() if beta is not None else None,
+                      float(eps), float(momentum), running_mean.data_ptr() if running_mean is not None else None,
+                      running_var.data_ptr() if running_var is not None else None, int(act), float(slope),
+                      stats.data_ptr(), y.data_ptr())
             with torch.cuda.device(z.device):
-                check(lib.ffb6d_bn_train_fwd(
-                    z.data_ptr(), B, Co, P, gamma.data_ptr() if gamma is not None else None,
-                    beta.data_ptr() if beta is not None else None, float(eps), float(momentum),
-                    running_mean.data_ptr() if running_mean is not None else None,
-                    running_var.data_ptr() if running_var is not None else None, int(act), float(slope),
-                    stats.data_ptr(), y.data_ptr(), ws.data_ptr(), nbytes, ops._stream(z.device)))
+                if group is None:
+                    check(lib.ffb6d_bn_train_fwd(z.data_ptr(), B, Co, P, *affine, ws.data_ptr(), nbytes,
+                                                 ops._stream(z.device)))
+                else:
+                    # [(sum z, sum z^2) per channel, local element count], summed over the group; the counts
+                    # may differ between ranks
+                    sums = torch.empty(2 * Co + 1, dtype=torch.float64, device=z.device)
+                    check(lib.ffb6d_bn_train_stats(z.data_ptr(), B, Co, P, sums.data_ptr(), ws.data_ptr(), nbytes,
+                                                   ops._stream(z.device)))
+                    sums[2 * Co] = float(B * P)
+                    dist.all_reduce(sums, group=group)
+                    count = float(sums[2 * Co])
+                    check(lib.ffb6d_bn_train_apply(z.data_ptr(), B, Co, P, sums.data_ptr(), count, *affine,
+                                                   ops._stream(z.device)))
         elif act == _ACT_RELU:
             y = torch.relu(z)
         elif act == _ACT_LEAKY:
@@ -93,6 +118,7 @@ class _ConvBnActTrain(torch.autograd.Function):
             y = z
         ctx.save_for_backward(x1, x2, w2d, z, stats, gamma)
         ctx.meta = (B, C1, C2, Co, P, int(act), float(slope), bool(has_bn), bias is not None, tuple(weight.shape))
+        ctx.sync = (group, count)
         return y
 
     @staticmethod
@@ -100,6 +126,7 @@ class _ConvBnActTrain(torch.autograd.Function):
     def backward(ctx, gy):
         x1, x2, w2d, z, stats, gamma = ctx.saved_tensors
         B, C1, C2, Co, P, act, slope, has_bn, has_bias, wshape = ctx.meta
+        group, count = ctx.sync
         gy = gy.contiguous()
         dev = z.device
         ggamma = gbeta = gbias = None
@@ -110,9 +137,18 @@ class _ConvBnActTrain(torch.autograd.Function):
                 gbeta = torch.empty(Co, dtype=torch.float32, device=dev)
                 nbytes = int(lib.ffb6d_bn_workspace_bytes(Co, P))
                 ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-                check(lib.ffb6d_bn_train_bwd(z.data_ptr(), gy.data_ptr(), stats.data_ptr(), B, Co, P, act, slope,
-                                             ggamma.data_ptr(), gbeta.data_ptr(), dz.data_ptr(), ws.data_ptr(), nbytes,
-                                             ops._stream(dev)))
+                if group is None:
+                    check(lib.ffb6d_bn_train_bwd(z.data_ptr(), gy.data_ptr(), stats.data_ptr(), B, Co, P, act, slope,
+                                                 ggamma.data_ptr(), gbeta.data_ptr(), dz.data_ptr(), ws.data_ptr(),
+                                                 nbytes, ops._stream(dev)))
+                else:
+                    sums = torch.empty(2 * Co, dtype=torch.float64, device=dev)
+                    check(lib.ffb6d_bn_train_bwd_stats(z.data_ptr(), gy.data_ptr(), stats.data_ptr(), B, Co, P, act,
+                                                       slope, sums.data_ptr(), ggamma.data_ptr(), gbeta.data_ptr(),
+                                                       ws.data_ptr(), nbytes, ops._stream(dev)))
+                    dist.all_reduce(sums, group=group)
+                    check(lib.ffb6d_bn_train_bwd_apply(z.data_ptr(), gy.data_ptr(), stats.data_ptr(), sums.data_ptr(),
+                                                       count, B, Co, P, act, slope, dz.data_ptr(), ops._stream(dev)))
             elif act != _ACT_NONE:
                 dz = torch.empty_like(z)
                 check(lib.ffb6d_act_bwd(z.data_ptr(), gy.data_ptr(), z.numel(), act, slope, dz.data_ptr(), ops._stream(dev)))
@@ -134,7 +170,16 @@ class _ConvBnActTrain(torch.autograd.Function):
             gx2 = _gemm(dz, None, w2d[:, C1:].t().contiguous()).reshape(x2.shape)
         if gamma is None:
             ggamma = None
-        return gx1, gx2, gw, gbias, ggamma, gbeta, None, None, None, None, None, None, None
+        return gx1, gx2, gw, gbias, ggamma, gbeta, None, None, None, None, None, None, None, None
+
+
+def _sync_group(bn):
+    """The process group a training-mode ``nn.SyncBatchNorm`` takes its statistics over, decided as
+    ``nn.SyncBatchNorm.forward`` decides; None for any other BatchNorm or when there is nothing to sync with."""
+    if not isinstance(bn, nn.SyncBatchNorm) or not (dist.is_available() and dist.is_initialized()):
+        return None
+    group = bn.process_group if bn.process_group is not None else dist.group.WORLD
+    return group if dist.get_world_size(group) > 1 else None
 
 
 class _BNWrap(nn.Sequential):
@@ -211,7 +256,8 @@ class _ConvBase(nn.Module):
             if bn.track_running_stats and bn.num_batches_tracked is not None:
                 bn.num_batches_tracked += 1
             return _ConvBnActTrain.apply(x, x2, conv.weight, None, bn.weight, bn.bias, bn.running_mean, bn.running_var,
-                                         bn.eps, bn.momentum if bn.momentum is not None else 0.1, self.act, self.slope, True)
+                                         bn.eps, bn.momentum if bn.momentum is not None else 0.1, self.act, self.slope, True,
+                                         _sync_group(bn))
         if need_grad and bn is None:
             return _ConvBnActTrain.apply(x, x2, conv.weight, conv.bias, None, None, None, None, 0.0, 0.0, self.act,
                                          self.slope, False)

@@ -301,6 +301,31 @@ int ffb6d_bn_train_fwd(const float *z, int64_t B, int64_t C, int64_t P, const fl
 int ffb6d_bn_train_bwd(const float *z, const float *grad_y, const float *stats, int64_t B, int64_t C, int64_t P,
                        int act, float negative_slope, float *grad_gamma, float *grad_beta, float *grad_z,
                        void *workspace, size_t workspace_bytes, ffb6d_stream_t stream);
+/* The same two passes split at their per-channel reductions, for synchronised BatchNorm across ranks
+ * (the reference converts every BatchNorm to SyncBN before DDP, train_ycb.py:568; torch.nn.SyncBatchNorm
+ * semantics).  Per layer and step:
+ *   ffb6d_bn_train_stats      sums [C][2] f64 = local (sum z, sum z^2)        -> all-reduce sums, and the counts
+ *   ffb6d_bn_train_apply      stats, y, running statistics from the global sums over count elements
+ *   ffb6d_bn_train_bwd_stats  sums [C][2] f64 = local (sum g', sum g' * xhat) -> all-reduce sums
+ *   ffb6d_bn_train_bwd_apply  grad_z from the global sums over the same count
+ * count is the global element count sum over ranks of B_r * P, >= the local B * P (every rank needs >= 1
+ * frame).  running_var takes the unbiased variance with the global count.  grad_gamma / grad_beta (may be
+ * NULL) are the LOCAL sums, as torch.nn.SyncBatchNorm returns them; DDP's gradient all-reduce averages them
+ * with every other parameter gradient.  The sums are added in the order of ffb6d_bn_train_fwd / _bwd and
+ * rounded as they are, so with the sums of one rank and count = B * P the split passes reproduce
+ * ffb6d_bn_train_fwd / ffb6d_bn_train_bwd bit for bit.  stats and workspace as above; sums 8-byte aligned. */
+int ffb6d_bn_train_stats(const float *z, int64_t B, int64_t C, int64_t P, double *sums,
+                         void *workspace, size_t workspace_bytes, ffb6d_stream_t stream);
+int ffb6d_bn_train_apply(const float *z, int64_t B, int64_t C, int64_t P, const double *sums, double count,
+                         const float *gamma, const float *beta, float eps, float momentum,
+                         float *running_mean, float *running_var, int act, float negative_slope,
+                         float *stats, float *y, ffb6d_stream_t stream);
+int ffb6d_bn_train_bwd_stats(const float *z, const float *grad_y, const float *stats, int64_t B, int64_t C,
+                             int64_t P, int act, float negative_slope, double *sums, float *grad_gamma,
+                             float *grad_beta, void *workspace, size_t workspace_bytes, ffb6d_stream_t stream);
+int ffb6d_bn_train_bwd_apply(const float *z, const float *grad_y, const float *stats, const double *sums,
+                             double count, int64_t B, int64_t C, int64_t P, int act, float negative_slope,
+                             float *grad_z, ffb6d_stream_t stream);
 /* grad_z = grad_y * act'(z) for a layer with an activation but no BatchNorm. */
 int ffb6d_act_bwd(const float *z, const float *grad_y, int64_t n, int act, float negative_slope, float *grad_z,
                   ffb6d_stream_t stream);

@@ -3,11 +3,13 @@
 fusion + heads (ffb6d_b200.model.FFB6DFusionNet: everything of FFB6D.forward except the ResNet/PSPNet image
 backbone, whose stage outputs are synthetic leaf tensors) under DistributedDataParallel, one process per GPU,
 NCCL gradient all-reduce -- the reference's recipe (train_ycb.py:536-539, 596-599).  BatchNorm statistics are per
-GPU (the reference additionally converts to apex SyncBN, train_ycb.py:568; BASELINE.json's north_star keeps NCCL
-"only for the DDP gradient allreduce", so the cross-rank statistics exchange is not part of this path).
+GPU by default; --sync-bn converts every BatchNorm with torch.nn.SyncBatchNorm.convert_sync_batchnorm before the DDP
+wrap, as the reference converts to SyncBN (train_ycb.py:568): with more than one GPU every BatchNorm layer then
+all-reduces its statistics in the forward and in the backward.
 
     python tools/train_bench.py --config 3                      (1 GPU)
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 tools/train_bench.py --config 3
+    ... tools/train_bench.py --config 3 --sync-bn               (global-batch BatchNorm statistics)
 
 Config 3: LineMOD-shaped (2 classes, 8 keypoints + centre), batch 8 per GPU, forward + backward.
 Config 4: YCB-shaped (22 classes), batch 4 per GPU, forward + backward + Adam step ("end-to-end train step").
@@ -31,6 +33,7 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--batch", type=int, default=0)
+    ap.add_argument("--sync-bn", action="store_true", help="convert every BatchNorm to torch.nn.SyncBatchNorm")
     ap.add_argument("--profile", action="store_true", help="print the per-kernel GPU time of one step (CUPTI) to stderr")
     args = ap.parse_args()
     import numpy as np
@@ -51,6 +54,8 @@ def main():
     N0 = 12288
     torch.manual_seed(0)
     model = FFB6DFusionNet(n_classes=n_classes, n_pts=N0, n_kps=n_kps).to(dev).train()
+    if args.sync_bn:
+        model = torch.nn.SyncBatchNorm.convert_sync_batchnorm(model)
     n_params = sum(p.numel() for p in model.parameters())
     net = torch.nn.parallel.DistributedDataParallel(model, device_ids=[local_rank], output_device=local_rank,
                                                     find_unused_parameters=False) if world > 1 else model
@@ -131,11 +136,12 @@ def main():
     if rank == 0:
         line = {"metric": "FFB6D point branch + fusion + heads, training step, points/s", "config": args.config,
                 "what": ("forward + backward" if args.config == 3 else "forward + backward + Adam step")
-                + ", DDP gradient all-reduce over NCCL" * (world > 1),
+                + ", DDP gradient all-reduce over NCCL" * (world > 1)
+                + ", SyncBatchNorm statistics all-reduce over NCCL" * (world > 1 and args.sync_bn),
                 "value": world * B * N0 * args.steps / (ms / 1e3), "unit": "points/s", "n_gpus": world,
                 "batch_per_gpu": B, "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms / args.steps,
                 "params": n_params, "grad_allreduce_bytes": 4 * n_params if world > 1 else 0, "loss": float(loss.detach()),
-                "finite": finite, "dtype": "f32", "data": "synthetic", "scaling": "weak"}
+                "finite": finite, "sync_bn": args.sync_bn, "dtype": "f32", "data": "synthetic", "scaling": "weak"}
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
